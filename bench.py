@@ -487,14 +487,14 @@ def _train_section(dev, calls, ndup, P, steps, V, peak):
 
 def _c3_section(dev, n_steps=6):
     """BASELINE config C3 on this GPU: the reference's OWN RtStereoHumanModel + loader + train_stage2.py:57-89 step (AMP,
-    GradScaler) from baseline/_ref against the drop-ins, 512^2 sources / 1024^2 render, batch 2 -- plain drop-ins and with
+    GradScaler) from oracle/_ref against the drop-ins, 512^2 sources / 1024^2 render, batch 2 -- plain drop-ins and with
     the GPSG_PATCH fused paths.  Stage split by CUDA events between the statements of the step; rasterizer kernel time from
     the library's own per-kernel events."""
     import tempfile
     import torch
     from gps_gaussian_b200 import _lib, harness, patch, synth_dataset
     if harness.staged_reference() is None:
-        return {"unavailable": "baseline/_ref not staged (build() stages it where /root/reference is mounted)"}
+        return {"unavailable": "oracle/_ref not staged (python oracle/build.py --reference <GPS-Gaussian checkout>)"}
     root = tempfile.mkdtemp(prefix="gpsg_c3_")
     synth_dataset.write_dataset(root, n_train=2, n_val=1, res=512, hr=True)
     out = {"config": "C3: reference RtStereoHumanModel (5 144 408 params), AMP + GradScaler, batch 2, 512^2 stereo pair -> "
@@ -539,13 +539,36 @@ def _c3_section(dev, n_steps=6):
     return out
 
 
+def dump_outputs(out_dir, colors, radii, num_rendered, budget=64 << 20):
+    """What the timed path handed its caller in the last step, as out_dir/<name>.npy: per view a fixed, seeded sample of
+    the rendered pixels (`color`, [V,3,n]) and of the Gaussians' screen radii (`radii`, [V,m]), the sampled indices, and
+    the tile-pair count.  Same arguments => same scenes and same samples, so two builds can be compared array by array.
+    Samples shrink with the number of views so that the files stay under `budget` bytes."""
+    import torch
+    V, (_, H, W), P = len(colors), tuple(colors[0].shape), min(int(r.numel()) for r in radii)
+    rng = np.random.default_rng(0)
+    n_pix = min(H * W, budget // 2 // (V * 3 * 4 + 8))
+    n_gau = min(P, budget // 4 // (V * 4 + 8))
+    pix = np.sort(rng.choice(H * W, n_pix, replace=False))
+    gau = np.sort(rng.choice(P, n_gau, replace=False))
+    pix_t, gau_t = torch.from_numpy(pix).to(colors[0].device), torch.from_numpy(gau).to(colors[0].device)
+    arrays = {"color": torch.stack([c.reshape(3, H * W).index_select(1, pix_t) for c in colors]).cpu().numpy(),
+              "pixel_index": pix.astype(np.float64),
+              "radii": torch.stack([r.index_select(0, gau_t) for r in radii]).float().cpu().numpy(),
+              "gaussian_index": gau.astype(np.float64),
+              "num_rendered": np.asarray(num_rendered, np.float64)}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def dict_copy(data):
     """Shallow per-view copy of a reference batch dict (the model writes its outputs into it)."""
     return {k: (dict(v) if isinstance(v, dict) else v) for k, v in data.items()}
 
 
 def run_c5(args, rank, world, local_rank):
-    """BASELINE config C5: stage-2 TRAINING data-parallel -- the reference's own model + step from baseline/_ref, 2 stereo
+    """BASELINE config C5: stage-2 TRAINING data-parallel -- the reference's own model + step from oracle/_ref, 2 stereo
     pairs of 1024^2 per GPU (2048^2 novel view, use_hr_img), ONE flat NCCL all-reduce (5 144 408 fp32 = 20.6 MB) between
     backward and unscale_ (train_stage2.py:83-85).  metric: pixels/s of source-pair pixels trained on (16 x 1024^2 per
     step at N=8), plus the exposed all-reduce time (step with all-reduce minus step without)."""
@@ -614,7 +637,7 @@ def run_c5(args, rank, world, local_rank):
         line = {"metric": "stage2_train_source_pixels_per_sec", "value": px / (ms * 1e-3), "unit": "pixels/s", "n_gpus": world,
                 "steps": args.steps, "warmup": max(3, args.warmup), "ms_per_step": ms, "higher_is_better": True, "scaling": "weak",
                 "vs_baseline": None, "dtype": "fp16 autocast nets + fp32 rasterizer (reference AMP)", "data": "synthetic",
-                "config": {"workload": f"C5: stage-2 training, reference RtStereoHumanModel from baseline/_ref, 2 pairs/GPU of {res}^2 "
+                "config": {"workload": f"C5: stage-2 training, reference RtStereoHumanModel from oracle/_ref, 2 pairs/GPU of {res}^2 "
                                        f"(render {2 * res}^2), global batch {2 * world}, flat NCCL all-reduce of 5144408 fp32 grads",
                            "fast_paths": "GPSG_PATCH fused paths" if args.patch else "plain drop-ins", "parallelism": f"dp{world}"},
                 "exposed_comm_ms": res_ms["with_allreduce_stages"].get("allreduce"),
@@ -648,6 +671,7 @@ def main():
     ap.add_argument("--train-c5", action="store_true", help="time data-parallel stage-2 training (C5) instead of the render")
     ap.add_argument("--c5-res", type=int, default=1024)
     ap.add_argument("--patch", action="store_true", help="C5: use the GPSG_PATCH fused paths")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the renders of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
 
@@ -728,6 +752,8 @@ def main():
     barrier()
     ms = e0.elapsed_time(e1)
     prof_overlapped = _lib.profile_read()
+    last_step = [(pr.color.clone(), pr.radii.clone(), pr.status()["num_rendered"]) for pr in planned] \
+        if args.dump_outputs else None
     clocks = sampler.stop()
     ms = shard.max_over_ranks(ms, dev)
     # Per-kernel durations for the roofline: with several streams the kernels of different views time-share the SMs, so
@@ -863,6 +889,10 @@ def main():
                 train, roof_b = _train_section(dev, calls, ndup, P, args.steps, V, peak)
             except Exception as exc:                               # never lose the headline line to an auxiliary measurement
                 train, roof_b = {"error": repr(exc)[:300]}, None
+
+    if last_step is not None:
+        dump_outputs(args.dump_outputs if world == 1 else os.path.join(args.dump_outputs, f"rank{rank}"),
+                     *zip(*last_step))
 
     if rank != 0:
         if world > 1:

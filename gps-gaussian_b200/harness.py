@@ -1,10 +1,10 @@
 """Run the UNMODIFIED reference scripts and model against the drop-ins (BASELINE config C3; VERDICT r1 item N1).
 
-The reference tree is staged once, byte for byte, into the git-ignored `baseline/_ref/` by `__graft_entry__.build()`
-(it travels to the GPU box with the snapshot like the built `.so`; it is never committed and nothing in the product
-imports it).  Everything here is harness: it builds the reference's own `RtStereoHumanModel`, feeds it the synthetic
-dataset through the reference's own `StereoHumanDataset`, and executes the optimisation step of
-/root/reference/train_stage2.py:57-89 -- with `gps-gaussian_b200/dropin` providing `diff_gaussian_rasterization`,
+The reference tree is staged, byte for byte, into the git-ignored `oracle/_ref/` by `oracle/build.py` when it finds a
+GPS-Gaussian checkout (`--reference DIR`, GPSG_REFERENCE_DIR, or its default location); it is never committed and
+nothing in the product imports it.  Everything here is harness: it builds the reference's own `RtStereoHumanModel`, feeds it the synthetic
+dataset through the reference's own `StereoHumanDataset`, and executes the optimisation step of the reference's
+train_stage2.py:57-89 -- with `gps-gaussian_b200/dropin` providing `diff_gaussian_rasterization`,
 `corr_sampler` and `yacs`.  Used by tests/test_c3_gpu.py and bench.py's `train_c3` block.
 """
 import os
@@ -15,20 +15,10 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
 DROPIN = os.path.join(HERE, "dropin")
-REF_SRC = "/root/reference"
-REF_STAGED = os.path.join(ROOT, "baseline", "_ref")
-
-
-def stage_reference(force=False):
-    """Copy /root/reference (read-only, only present in the build container) to baseline/_ref. Returns the staged path,
-    or None when neither the source nor an earlier staging exists."""
-    marker = os.path.join(REF_STAGED, "train_stage2.py")
-    if os.path.isdir(REF_SRC) and (force or not os.path.exists(marker)):
-        if os.path.isdir(REF_STAGED):
-            shutil.rmtree(REF_STAGED)
-        os.makedirs(os.path.dirname(REF_STAGED), exist_ok=True)
-        shutil.copytree(REF_SRC, REF_STAGED, ignore=shutil.ignore_patterns(".git", "__pycache__", "*.pyc"))
-    return REF_STAGED if os.path.exists(marker) else None
+REF_STAGED = os.path.join(ROOT, "oracle", "_ref")
+if ROOT not in sys.path:
+    sys.path.insert(0, ROOT)
+from oracle.build import make_writable  # noqa: E402
 
 
 def staged_reference():
@@ -39,7 +29,7 @@ def add_reference_to_path():
     """dropin first (so `diff_gaussian_rasterization`, `corr_sampler`, `yacs` resolve to ours), then the staged tree."""
     ref = staged_reference()
     if ref is None:
-        raise FileNotFoundError("baseline/_ref is not staged: run __graft_entry__.build() where /root/reference is mounted")
+        raise FileNotFoundError("oracle/_ref is not staged: run python oracle/build.py --reference <GPS-Gaussian checkout>")
     for p in (ref, DROPIN, ROOT):
         if p in sys.path:
             sys.path.remove(p)
@@ -69,10 +59,11 @@ def make_workdir(path, data_root, **cfg):
     cwd and write experiments/ into it) with our config/stage2.yaml in place of the placeholder one."""
     ref = staged_reference()
     if ref is None:
-        raise FileNotFoundError("baseline/_ref is not staged")
+        raise FileNotFoundError("oracle/_ref is not staged")
     if os.path.isdir(path):
         shutil.rmtree(path)
     shutil.copytree(ref, path)
+    make_writable(path)
     with open(os.path.join(path, "config", "stage2.yaml"), "w") as f:
         f.write(stage2_yaml(data_root, **cfg))
     return path

@@ -1,8 +1,8 @@
 """BASELINE config C3 on hardware: the reference's OWN stage-2 model, loader and optimisation step against the drop-ins.
 
 Only `gps-gaussian_b200/dropin` (-> `diff_gaussian_rasterization`, `corr_sampler`, `yacs`) and the staged, unmodified
-reference tree `baseline/_ref` (git-ignored; staged by `__graft_entry__.build()`; ships with the gpurun snapshot) are
-put on `sys.path`.  Checked, per VERDICT r1 "next round" item 1:
+reference tree `oracle/_ref` (git-ignored; staged by `build()`, see oracle/build.py) are put on `sys.path`.  The
+repository does not carry the reference's sources, so these tests skip where nothing was staged.  Checked, per VERDICT r1 "next round" item 1:
   (a) train_stage2.py:57-89 executed statement for statement (AMP + GradScaler): finite loss, finite gradients on every
       parameter, the scaler does not skip the step;
   (b) `img_pred` equals the CPU-oracle render of the Gaussians the network produced, within the rasterizer parity bound;
@@ -25,7 +25,7 @@ from gps_gaussian_b200 import harness
 
 pytestmark = [pytest.mark.gpu,
               pytest.mark.skipif(harness.staged_reference() is None,
-                                 reason="baseline/_ref not staged (run __graft_entry__.build() where /root/reference exists)")]
+                                 reason="oracle/_ref not staged (python oracle/build.py --reference <GPS-Gaussian checkout>)")]
 
 RES = 512
 
@@ -158,7 +158,7 @@ def test_c3_patched_fast_paths_give_the_same_step(dataset):
 @pytest.mark.parametrize("patched", [False, True])
 def test_reference_scripts_run_unmodified(dataset, tmp_path, patched):
     """(d): `python train_stage2.py` (3 steps, batch 2, AMP) then `python test_view_interp.py` on the checkpoint it
-    saved, cwd = a working copy of baseline/_ref whose only change is config/stage2.yaml's data_root / num_steps."""
+    saved, cwd = a working copy of oracle/_ref whose only change is config/stage2.yaml's data_root / num_steps."""
     work = harness.make_workdir(str(tmp_path / "work"), dataset, src_res=RES, num_steps=3, batch_size=2)
     for name in ("train_stage2.py", "test_view_interp.py", "lib/GaussianRender.py", "core/corr.py"):
         with open(os.path.join(work, name), "rb") as a, open(os.path.join(harness.REF_STAGED, name), "rb") as b:
