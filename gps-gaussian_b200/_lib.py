@@ -112,6 +112,11 @@ lib.gpsg_unproject_forward.restype = _i
 lib.gpsg_unproject_forward.argtypes = [_i, _vp, _i, _i, _vp, _vp, _i64, _vp, _vp, _i, _vp, _vp, _vp, _vp, _vp]
 lib.gpsg_unproject_backward.restype = _i
 lib.gpsg_unproject_backward.argtypes = [_i, _vp, _i, _i, _vp, _vp, _i64, _vp, _vp, _i, _vp, _vp, _vp, _vp, _vp]
+lib.gpsg_flow2render_workspace_bytes.restype = _sz
+lib.gpsg_flow2render_workspace_bytes.argtypes = [_i, _i]
+lib.gpsg_flow2render.restype = _i
+lib.gpsg_flow2render.argtypes = [_i, _vp, _i, _i, _i, _i, _pp, _pp, C.POINTER(C.c_int64), _pp, _pp, _i, _pp, _pp, _pp, _vp,
+                                 _vp, _sz, _vp, _vp]
 lib.gpsg_l1_ssim_workspace_bytes.restype = _sz
 lib.gpsg_l1_ssim_workspace_bytes.argtypes = [_i, _i, _i]
 lib.gpsg_l1_ssim_forward.restype = _i
@@ -132,7 +137,8 @@ EXPORTED = ["gpsg_last_error", "gpsg_version", "gpsg_rasterize_forward", "gpsg_r
             "gpsg_raster_binning_bytes", "gpsg_raster_image_bytes", "gpsg_raster_status_ptr",
             "gpsg_rasterize_forward_planned", "gpsg_rasterize_forward_maps", "gpsg_rasterize_forward_maps_planned", "gpsg_rasterize_forward_maps_begin", "gpsg_rasterize_forward_maps_finish",
             "gpsg_rasterize_backward_maps_workspace_bytes",
-            "gpsg_rasterize_backward_maps", "gpsg_unproject_forward", "gpsg_unproject_backward", "gpsg_l1_ssim_workspace_bytes", "gpsg_l1_ssim_forward",
+            "gpsg_rasterize_backward_maps", "gpsg_unproject_forward", "gpsg_unproject_backward", "gpsg_flow2render_workspace_bytes",
+            "gpsg_flow2render", "gpsg_l1_ssim_workspace_bytes", "gpsg_l1_ssim_forward",
             "gpsg_l1_ssim_backward", "gpsg_set_corr_build", "gpsg_profile_enable",
             "gpsg_profile_read",
             "gpsg_profile_stage_name"]

@@ -4,7 +4,8 @@
 
 Output: gps-gaussian_b200/lib/libgpsg_sm100.so (git-ignored; travels to the GPU box with gpurun).
 raster_preprocess.cu is compiled with -fmad=false (see its header): the fp32 op order that decides
-radii / tile rectangles must not be FMA-contracted.
+radii / tile rectangles must not be FMA-contracted.  point_splat.cu likewise: the stage-1 preview's pixel and
+inverse depth are replayed bit for bit by the CPU oracle.
 """
 import os
 import subprocess
@@ -31,6 +32,7 @@ SOURCES = {
     "sh.cu": [],
     "unproject.cu": [],
     "loss.cu": [],
+    "point_splat.cu": ["-fmad=false"],
 }
 
 

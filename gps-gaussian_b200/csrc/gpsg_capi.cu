@@ -691,6 +691,37 @@ int gpsg_unproject_backward(int device, void* stream_, int B, int S, const float
                                 dL_ddepth, dL_dflow, (cudaStream_t)stream_);
 }
 
+size_t gpsg_flow2render_workspace_bytes(int B, int res) {
+    return (B > 0 && res > 0) ? (size_t)B * res * res * sizeof(unsigned long long) : 0;
+}
+
+int gpsg_flow2render(int device, void* stream_, int B, int bs, int S, int res, const float* const* flow_pred,
+                     const float* const* mask, const int64_t* mask_batch_stride, const float* const* intr,
+                     const float* const* extr, int extr_rows, const float* const* ref_intr, const float* const* Tf_x,
+                     const float* const* img, const float* novel_calib, void* workspace, size_t workspace_bytes,
+                     float* out_color, float* out_inv_depth) {
+    GPSG_REQUIRE(B > 0 && res > 0, "flow2render: empty batch or image");
+    GPSG_REQUIRE(bs >= 0 && bs <= B, "flow2render: bs must be in [0, B]");
+    GPSG_REQUIRE(S == res, "flow2render: source maps must be res x res");
+    GPSG_REQUIRE(2 * (int64_t)S * S + 1 < ((int64_t)1 << 32), "flow2render: 2*S^2 + 1 must fit the 32-bit point id");
+    GPSG_REQUIRE(extr_rows >= 3, "flow2render: extr needs >= 3 rows");
+    GPSG_REQUIRE(flow_pred && mask && mask_batch_stride && intr && extr && ref_intr && Tf_x && img && novel_calib &&
+                 workspace && out_color, "NULL pointer");
+    FlowSplatViews in;
+    for (int v = 0; v < 2; ++v) {
+        GPSG_REQUIRE(flow_pred[v] && mask[v] && intr[v] && extr[v] && ref_intr[v] && Tf_x[v] && img[v],
+                     "NULL per-view pointer");
+        GPSG_REQUIRE(mask_batch_stride[v] >= (int64_t)S * S, "flow2render: mask batch stride < S^2");
+        in.flow[v] = flow_pred[v]; in.mask[v] = mask[v]; in.mask_bs[v] = mask_batch_stride[v]; in.intr[v] = intr[v];
+        in.extr[v] = extr[v]; in.ref_intr[v] = ref_intr[v]; in.Tf_x[v] = Tf_x[v]; in.img[v] = img[v];
+    }
+    in.extr_rows = extr_rows;
+    GPSG_REQUIRE(workspace_bytes >= gpsg_flow2render_workspace_bytes(B, res), "flow2render: workspace too small");
+    GPSG_REQUIRE(((uintptr_t)workspace & 7) == 0, "flow2render: workspace must be 8-byte aligned");
+    GPSG_CUDA(cudaSetDevice(device));
+    return launch_flow2render(B, bs, S, res, in, novel_calib, workspace, out_color, out_inv_depth, (cudaStream_t)stream_);
+}
+
 size_t gpsg_l1_ssim_workspace_bytes(int planes, int H, int W) {
     return (planes > 0 && H > 0 && W > 0) ? l1_ssim_workspace_bytes(planes, H, W) : 256;
 }

@@ -181,8 +181,15 @@ int launch_unproject_fwd(int B, int S, const float* flow, const float* mask, int
 int launch_unproject_bwd(int B, int S, const float* depth, const float* mask, int64_t mask_bs, const float* intr,
                          const float* extr, int extr_rows, const float* ref_intr, const float* Tf_x,
                          const float* dL_dxyz, const float* dL_ddepth, float* dL_dflow, cudaStream_t stream);
+// point_splat.cu (compiled with -fmad=false: the CPU oracle replays its fp32 op order)
+struct FlowSplatViews {   // per source view v in {0: lmain, 1: rmain}; passed by value to the kernel
+    const float* flow[2]; const float* mask[2]; int64_t mask_bs[2]; const float* intr[2]; const float* extr[2];
+    int extr_rows; const float* ref_intr[2]; const float* Tf_x[2]; const float* img[2];
+};
+int launch_flow2render(int B, int bs, int S, int res, const FlowSplatViews& in, const float* calib, void* zbuf,
+                       float* color, float* inv_depth, cudaStream_t stream);
 // corr.cu
-int corr_build_mode();            // 0 = tcgen05 when possible, 1 = FFMA kernels
+int corr_build_mode();           // 0 = tcgen05 when possible, 1 = FFMA kernels
 void set_corr_build_mode(int m);
 int launch_corr_fwd(int dtype, int B, int H, int W1, int W2, const void* vol, int64_t sb, int64_t sh, int64_t sw1,
                     const float* coords, int64_t csb, int r, void* out, cudaStream_t stream);

@@ -4,28 +4,9 @@
 // One kernel forward (depth, xyz, pts_valid) and one backward (d xyz [+ d depth] -> d flow).  HBM-bound:
 // forward reads 8 B and writes 17 B per pixel.
 #include "gpsg_internal.cuh"
+#include "unproject_math.cuh"
 
 namespace gpsg {
-
-// per batch item: K (fx, fy, cx, cy), R (3x3 row-major), t (3), offset = ref_cx - cx, 1/Tf_x sign folded
-struct UnprojCam { float fx, fy, cx, cy, R[9], t[3], offset, tfx; };
-
-__device__ __forceinline__ UnprojCam load_cam(const float* intr, const float* extr, int extr_row_stride,
-                                              const float* ref_intr, const float* Tf_x, int b) {
-    UnprojCam c;
-    const float* K = intr + 9 * (size_t)b;
-    const float* E = extr + (size_t)b * extr_row_stride * 4;     // [rows>=3, 4]
-    c.fx = K[0]; c.fy = K[4]; c.cx = K[2]; c.cy = K[5];
-#pragma unroll
-    for (int r = 0; r < 3; ++r) {
-#pragma unroll
-        for (int k = 0; k < 3; ++k) c.R[3 * r + k] = E[4 * r + k];
-        c.t[r] = E[4 * r + 3];
-    }
-    c.offset = ref_intr[9 * (size_t)b + 2] - K[2];
-    c.tfx = Tf_x[b];
-    return c;
-}
 
 __global__ void __launch_bounds__(256) unproject_forward_kernel(int B, int S, const float* __restrict__ flow,
                                                                 const float* __restrict__ mask, int64_t mask_bs,
@@ -42,24 +23,13 @@ __global__ void __launch_bounds__(256) unproject_forward_kernel(int B, int S, co
     const int64_t pix = idx - (int64_t)b * S2;
     const int v = (int)(pix / S), u = (int)(pix % S);
     const UnprojCam c = load_cam(intr, extr, extr_rows, ref_intr, Tf_x, b);
-    // flow2depth: depth = -(offset - flow) / Tf_x * mask
-    const float disparity = c.offset - flow[idx];
-    float d = -disparity / c.tfx;
-    d *= mask[(size_t)b * mask_bs + pix];
+    float p[3];
+    const float d = unproject_pixel(c, flow[idx], mask[(size_t)b * mask_bs + pix], u, v, p);
     depth[idx] = d;
     valid[idx] = d != 0.0f;
-    // depth2pc: inverse-depth parameterisation, pixel centres at +0.5
-    const float z = 1.0f / (d + 1e-8f);
-    const float px = (((float)u + 0.5f) - c.cx) * z / c.fx;
-    const float py = (((float)v + 0.5f) - c.cy) * z / c.fy;
-    // pts = R^T p - R^T t
     float* o = xyz + 3 * idx;
 #pragma unroll
-    for (int k = 0; k < 3; ++k) {
-        const float rp = c.R[k] * px + c.R[3 + k] * py + c.R[6 + k] * z;
-        const float rt = c.R[k] * c.t[0] + c.R[3 + k] * c.t[1] + c.R[6 + k] * c.t[2];
-        o[k] = rp - rt;
-    }
+    for (int k = 0; k < 3; ++k) o[k] = p[k];
 }
 
 __global__ void __launch_bounds__(256) unproject_backward_kernel(int B, int S, const float* __restrict__ depth,

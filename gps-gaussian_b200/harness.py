@@ -37,13 +37,14 @@ def add_reference_to_path():
     return ref
 
 
-def stage2_yaml(data_root, src_res=512, num_steps=3, batch_size=2, corr_implementation=None, use_processed_data=True):
+def stage2_yaml(data_root, src_res=512, num_steps=3, batch_size=2, corr_implementation=None, use_processed_data=True,
+                stage1_ckpt=None):
     """The reference's own config/stage2.yaml with only the user-facing knobs changed (data_root and stage1_ckpt are
-    placeholders upstream: 'PATH/TO/...')."""
+    placeholders upstream: 'PATH/TO/...'; `stage1_ckpt` = a checkpoint train_stage1.py wrote, else "None")."""
     import yaml
     with open(os.path.join(staged_reference(), "config", "stage2.yaml")) as f:
         y = yaml.safe_load(f)
-    y["stage1_ckpt"] = "None"
+    y["stage1_ckpt"] = "None" if stage1_ckpt is None else str(stage1_ckpt)
     y["num_steps"] = int(num_steps)
     y["batch_size"] = int(batch_size)
     y["dataset"]["src_res"] = int(src_res)
@@ -54,9 +55,26 @@ def stage2_yaml(data_root, src_res=512, num_steps=3, batch_size=2, corr_implemen
     return yaml.safe_dump(y, sort_keys=False)
 
 
-def make_workdir(path, data_root, **cfg):
+def stage1_yaml(data_root, src_res=512, num_steps=3, batch_size=2, eval_freq=1, loss_freq=1, use_processed_data=True):
+    """The reference's own config/stage1.yaml (fp32: mixed_precision False) with only the user-facing knobs changed.
+    train_stage1.py validates over int(len(val_loader) / 200) batches of 2 (:36-37): the dataset needs >= 2 val samples."""
+    import yaml
+    with open(os.path.join(staged_reference(), "config", "stage1.yaml")) as f:
+        y = yaml.safe_load(f)
+    y["num_steps"] = int(num_steps)
+    y["batch_size"] = int(batch_size)
+    y["dataset"]["src_res"] = int(src_res)
+    y["dataset"]["data_root"] = str(data_root)
+    y["dataset"]["use_processed_data"] = bool(use_processed_data)
+    y["record"]["eval_freq"] = int(eval_freq)
+    y["record"]["loss_freq"] = int(loss_freq)
+    return yaml.safe_dump(y, sort_keys=False)
+
+
+def make_workdir(path, data_root, stage1=None, **cfg):
     """A working copy of the staged tree (the scripts resolve 'config/stage2.yaml', 'core', 'lib', ... relative to the
-    cwd and write experiments/ into it) with our config/stage2.yaml in place of the placeholder one."""
+    cwd and write experiments/ into it) with our config/stage2.yaml in place of the placeholder one, and, when `stage1`
+    (a dict of stage1_yaml keywords) is given, our config/stage1.yaml too."""
     ref = staged_reference()
     if ref is None:
         raise FileNotFoundError("oracle/_ref is not staged")
@@ -66,6 +84,9 @@ def make_workdir(path, data_root, **cfg):
     make_writable(path)
     with open(os.path.join(path, "config", "stage2.yaml"), "w") as f:
         f.write(stage2_yaml(data_root, **cfg))
+    if stage1 is not None:
+        with open(os.path.join(path, "config", "stage1.yaml"), "w") as f:
+            f.write(stage1_yaml(data_root, **stage1))
     return path
 
 

@@ -12,6 +12,13 @@ installs a post-import hook that, right after the reference executes those two m
 so `from core.corr import CorrBlockFast1D` (core/raft_stereo_human.py:6) and `from lib.GaussianRender import pts2render`
 (train_stage2.py:15, test_view_interp.py:15) pick ours up.  Same names, signatures and results (tests/test_c3_gpu.py runs
 the stage-2 step both ways).  `install()` / `uninstall()` do the same for modules that are already imported.
+
+lib.TaichiRender (train_stage1.py:16) cannot be patched after it executes: it imports `taichi` and calls
+`ti.init(ti.cuda)` at import time, and taichi is not installable here.  It is SUBSTITUTED instead: while the hook is
+installed, `import lib.TaichiRender` yields a module whose `TaichiRenderBatch` is gps_gaussian_b200.TaichiRender's (the
+sm_100a preview splat), without running the reference file.  A real lib.TaichiRender that is already imported (taichi
+present) gets its attribute rebound like the other targets.  `uninstall()` drops the substitute from sys.modules, so the
+next import runs the reference module again (and fails again without taichi).
 """
 import importlib.abc
 import importlib.machinery
@@ -41,7 +48,26 @@ def _patch_render(mod):
     _set(mod, "pts2render", ours.pts2render)
 
 
-_TARGETS = {"core.corr": _patch_corr, "lib.GaussianRender": _patch_render}
+def _patch_taichi(mod):
+    from gps_gaussian_b200 import TaichiRender as ours
+    _set(mod, "TaichiRenderBatch", ours.TaichiRenderBatch)
+
+
+_TARGETS = {"core.corr": _patch_corr, "lib.GaussianRender": _patch_render, "lib.TaichiRender": _patch_taichi}
+_SUBSTITUTE = {"lib.TaichiRender"}       # never executed: the hook builds the module from ours
+_MARK = "__gpsg_substitute__"
+
+
+class _SubstituteLoader(importlib.abc.Loader):
+    def __init__(self, hook):
+        self._hook = hook
+
+    def create_module(self, spec):
+        return None                      # default module object
+
+    def exec_module(self, module):
+        setattr(module, _MARK, True)
+        self._hook(module)
 
 
 class _PatchingLoader(importlib.abc.Loader):
@@ -61,6 +87,8 @@ class _Finder(importlib.abc.MetaPathFinder):
         hook = _TARGETS.get(name)
         if hook is None:
             return None
+        if name in _SUBSTITUTE:
+            return importlib.machinery.ModuleSpec(name, _SubstituteLoader(hook), origin="gps_gaussian_b200 substitute")
         for finder in sys.meta_path:
             if finder is self or not hasattr(finder, "find_spec"):
                 continue
@@ -88,9 +116,16 @@ def uninstall():
         sys.meta_path.remove(_FINDER)
     for (modname, attr), orig in list(_ORIG.items()):
         mod = sys.modules.get(modname)
-        if mod is not None and orig is not None:
+        if mod is not None and orig is not None and not getattr(mod, _MARK, False):
             setattr(mod, attr, orig)
     _ORIG.clear()
+    for name in _SUBSTITUTE:
+        mod = sys.modules.get(name)
+        if mod is not None and getattr(mod, _MARK, False):
+            del sys.modules[name]
+            parent, _, child = name.rpartition(".")
+            if getattr(sys.modules.get(parent), child, None) is mod:
+                delattr(sys.modules[parent], child)
 
 
 def active():

@@ -221,3 +221,57 @@ def corr_inputs(B=2, D=192, H=64, W=64, seed=SEED, dtype=np.float32):
     ys = np.broadcast_to(np.arange(H, dtype=np.float32)[:, None], (B, H, W))
     coords = np.stack([xs + rng.normal(0, 6.0, (B, H, W)).astype(np.float32), ys], 1).astype(np.float32)
     return f1, f2, np.ascontiguousarray(coords)
+
+
+def novel_calib_for_show(intr, extr, ratio=0.5):
+    """data['novel_view'] intr[B,3,3] / extr[B,3,4] (float32) as reference lib/utils.py:57-84 builds them for the
+    stage-1 preview: scipy Slerp of the two source rotations, linear translation and intrinsics."""
+    from scipy.spatial.transform import Rotation, Slerp
+    K_out, E_out = [], []
+    for b in range(intr.shape[1]):
+        i0, i1 = intr[0, b], intr[1, b]
+        e0, e1 = extr[0, b], extr[1, b]
+        rot = Slerp([0, 1], Rotation.from_matrix(np.stack([e0[:3, :3], e1[:3, :3]])))(ratio)
+        pose = np.diag([1.0, 1.0, 1.0, 1.0]).astype(np.float32)
+        pose[:3, :3] = rot.as_matrix()
+        pose[:3, 3] = ((1.0 - ratio) * e0 + ratio * e1)[:3, 3]
+        E_out.append(pose[:3, :])
+        K_out.append((1.0 - ratio) * i0 + ratio * i1)
+    return np.array(K_out, np.float32), np.array(E_out, np.float32)
+
+
+def stage1_batch(res=256, B=2, seed=SEED, ratio=0.5, flow_noise=0.05):
+    """A synthetic stage-1 validation batch as train_stage1.py:96-100 hands it to TaichiRenderBatch.flow2render: per
+    source view (lmain, rmain: the ring cameras at -/+11.25 deg) flow_pred[B,1,S,S] (the capsule's inverse depth turned
+    into disparity flow, plus seeded noise), mask[B,1,S,S], intr / ref_intr [B,3,3], extr[B,4,4], Tf_x[B], img[B,3,S,S]
+    in [-1,1]; and data['novel_view'] intr / extr from novel_calib_for_show.  All float32 numpy."""
+    rng = np.random.default_rng(seed)
+    names = ("lmain", "rmain")
+    out = {n: {k: [] for k in ("flow_pred", "mask", "intr", "extr", "ref_intr", "Tf_x", "img")} for n in names}
+    v, u = np.meshgrid(np.arange(res) + 0.5, np.arange(res) + 0.5, indexing="ij")
+    for _ in range(B):
+        radius = 0.425 * float(rng.uniform(0.9, 1.05))
+        phase = float(rng.uniform(0, 6.28))
+        tfx = -0.6 * res * float(rng.uniform(0.95, 1.05))              # depth = (flow - offset) / Tf_x
+        for name, ang in zip(names, (-11.25, 11.25)):
+            K, E = ring_camera(ang, res)
+            z = _capsule_depth(K, E, res, radius, radius, 1.8 - radius)
+            hit = z > 0
+            inv = np.where(hit, 1.0 / np.maximum(z, 1e-6), 0.0)
+            Kr = K.copy()
+            Kr[0, 2] += 0.1 * res
+            offset = Kr[0, 2] - K[0, 2]
+            flow = offset + inv * tfx + flow_noise * rng.standard_normal((res, res))
+            pc = np.stack([(u - K[0, 2]) * z / K[0, 0], (v - K[1, 2]) * z / K[1, 1], z], -1)
+            xyz = (pc - E[:, 3]) @ E[:, :3]
+            img = np.where(hit[..., None], 0.8 * np.sin(xyz @ np.array([[9.0, 5.0, 7.0], [4.0, 11.0, 6.0],
+                                                                         [7.0, 3.0, 10.0]]).T + phase), -1.0)
+            d = out[name]
+            d["flow_pred"].append(flow[None]); d["mask"].append(hit[None].astype(np.float64))
+            d["intr"].append(K); d["extr"].append(np.vstack([E, [0, 0, 0, 1]])); d["ref_intr"].append(Kr)
+            d["Tf_x"].append(tfx); d["img"].append(img.transpose(2, 0, 1))
+    data = {n: {k: np.ascontiguousarray(np.array(a, np.float32)) for k, a in out[n].items()} for n in names}
+    K_n, E_n = novel_calib_for_show(np.stack([data[n]["intr"] for n in names]),
+                                    np.stack([data[n]["extr"] for n in names]), ratio)
+    data["novel_view"] = {"intr": K_n, "extr": E_n}
+    return data

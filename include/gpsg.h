@@ -231,6 +231,27 @@ GPSG_API int gpsg_unproject_backward(int device, void* stream, int B, int S, con
                                      const float* ref_intr, const float* Tf_x, const float* dL_dxyz,
                                      const float* dL_ddepth, float* dL_dflow);
 
+/* ---- stage-1 validation preview: replaces TaichiRenderBatch.flow2render (reference lib/TaichiRender.py:26-60) ----------
+ * Per source view v in {0: lmain, 1: rmain} (pointer arrays of 2, like the *_maps entries): flow_pred[v][B,1,S,S],
+ * mask[v] (channel 0 of [B,C,S,S]; mask_batch_stride[v], HOST array of 2, in elements), intr[v][B,3,3],
+ * extr[v][B,extr_rows>=3,4], ref_intr[v][B,3,3], Tf_x[v][B], img[v][B,3,S,S] in [-1,1].  novel_calib[B,3,4] = K E of the
+ * novel camera.  Each pixel with depth != 0 is unprojected (as gpsg_unproject_forward), projected into the novel camera
+ * (x, y pixel coordinates; inv = 1/(z + 1e-8)) and splatted onto pixel (clamp(trunc x), clamp(trunc y)) -- off-screen
+ * points land on the border, as upstream -- keeping the point with the largest inv >= 0, the last one in (view, pixel)
+ * order on ties.  That is the sequential reading of upstream's racy atomic_max kernel; the result is deterministic.
+ * Only samples b < bs are rendered (upstream's Taichi field has bs rows); the others stay background.
+ * out_color[B,3,res,res] = the winner's raw img value, -1 where no point landed; out_inv_depth[B,res,res] (optional,
+ * may be NULL) = its inv, 0 where none.  Requires S == res, bs <= B and 2*S*S + 1 < 2^32.
+ * workspace (>= gpsg_flow2render_workspace_bytes(B, res), 8-byte aligned) holds the z-buffer of 64-bit keys
+ * (inv bits << 32 | v*S*S + pixel + 1; 0 = no point), left in place after the call.
+ * One memset and two kernel launches; no host synchronisation. */
+GPSG_API size_t gpsg_flow2render_workspace_bytes(int B, int res);
+GPSG_API int gpsg_flow2render(int device, void* stream, int B, int bs, int S, int res, const float* const* flow_pred,
+                              const float* const* mask, const int64_t* mask_batch_stride, const float* const* intr,
+                              const float* const* extr, int extr_rows, const float* const* ref_intr,
+                              const float* const* Tf_x, const float* const* img, const float* novel_calib,
+                              void* workspace, size_t workspace_bytes, float* out_color, float* out_inv_depth);
+
 /* ---- fused photometric loss on the rendered image (SURVEY.md 8f-4) -----------------------------------------------
  * replaces  0.8 * l1_loss(img, gt) + 0.2 * (1 - ssim(img, gt))  (train_stage2.py:70-72; lib/loss.py:35-72: 11x11 Gaussian
  * window sigma 1.5, zero padding, C1 = 0.01^2, C2 = 0.03^2, means over all planes*H*W elements) and its autograd.
